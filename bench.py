@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's config.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 metric : stereo pairs/sec for "MS features + cost volume + soft-argmin" at 540x960,
          D=192 (BASELINE.json configs[1]: SceneFlow-shaped batch of 8 pairs per GPU).
@@ -229,6 +229,8 @@ def run_ours(args):
     ms_res, prof = timed(step_resident, args.steps, args.warmup, profile=True)
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, feats, disp)
     ms_e2e, _ = timed(step_e2e, args.steps, min(args.warmup, 3), drain=drain_e2e)
 
     # soft-argmin kernel alone (for the per-kernel breakdown)
@@ -315,6 +317,24 @@ def run_ours(args):
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_FEATURE_SAMPLES = 1 << 22
+
+
+def dump_outputs(out_dir, feats, disp):
+    """Writes what the last timed step returned, for comparing two builds output for output:
+    disparity.npy, the whole [8,540,960] soft-argmin result, and ms_features_sample.npy, the MS feature
+    volume [8,8,192,540,960] (25.5 GB) at DUMP_FEATURE_SAMPLES voxels drawn with a fixed seed, in
+    ascending flat-index order.  Both float32, 33 MB in all."""
+    import numpy as np
+    import torch
+    n = feats.numel()
+    idx = np.sort(np.random.default_rng(0).integers(0, n, DUMP_FEATURE_SAMPLES))
+    sample = feats.reshape(-1).index_select(0, torch.from_numpy(idx).to(feats.device))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "disparity.npy"), disp.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "ms_features_sample.npy"), sample.float().cpu().numpy())
 
 
 def slab_config_m(dev, rank, world, steps=3, warmup=2):
@@ -583,7 +603,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--cpu-sample", default=None, help="internal: time one reference step with this oracle/_ref build")
     ap.add_argument("--budget", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's outputs to DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.cpu_sample:
         print(json.dumps(_cpu_sample_one(args.cpu_sample, args.budget)))
         return

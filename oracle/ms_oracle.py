@@ -369,10 +369,11 @@ def down_sampling_input(ds_scale, imgl, imgr):
     return out[0], out[1]
 
 
-def generate_test_cbmv(imgl, imgr, encoder_ds=64, maxdisp=192, args_dict=None, is_left_only=True):
+def generate_test_cbmv(imgl, imgr, encoder_ds=64, maxdisp=192, args_dict=None, is_left_only=True, mtc=MTC,
+                       fte=FTE):
     """cbmv_generator.py:727-861 on two uint8 gray images (the reference reads them with
     cv2.imread(name, 0)).  ds_scale > 1 goes through down_sampling_input (rescale_antialiased: pinned to
-    scipy.ndimage, not to skimage itself -- see there).
+    scipy.ndimage, not to skimage itself -- see there).  `mtc`/`fte` as in get_costs.
     Returns (features float32 [C, D, crop_h, crop_w], h, w, crop_h, crop_w)."""
     ad = dict(censw=11, nccw=3, sadw=5, sobelw=5, cens_sigma=128.0, ncc_sigma=0.02, sad_sigma=20000.0,
               sobel_sigma=20000.0, ds_scale=1)
@@ -389,9 +390,9 @@ def generate_test_cbmv(imgl, imgr, encoder_ds=64, maxdisp=192, args_dict=None, i
     L = np.ascontiguousarray(np.pad(pl, ((10, 10), (10, 10)), "constant").astype(np.uint8))
     R = np.ascontiguousarray(np.pad(pr, ((10, 10), (10, 10)), "constant").astype(np.uint8))
     costs = get_costs(L, R, maxdisp // ds, ad["censw"], ad["nccw"], ad["sadw"], ad["sobelw"],
-                      10, 10, 10)
+                      10, 10, 10, mtc=mtc, fte=fte)
     fn = extract_features_left if is_left_only else extract_features_lr
-    f = fn(*costs, cens_sigma=ad["cens_sigma"], ncc_sigma=ad["ncc_sigma"], sad_sigma=ad["sad_sigma"])
+    f = fn(*costs, cens_sigma=ad["cens_sigma"], ncc_sigma=ad["ncc_sigma"], sad_sigma=ad["sad_sigma"], fte=fte)
     return f, h, w, crop_h, crop_w
 
 

@@ -15,6 +15,9 @@ GPU box like the compiled reference).  The generator's other imports are stubbed
 matplotlib are absent from this image (only used by down_sampling_input and the plot helpers),
 `..pfmutil` / `..funcs_utili` are the reference's PFM reader and plotting module.
 
+Where neither copy exists, restated_generator() gives the oracle's restatement of the same glue behind
+the same interface, and write_standin_package() a `src` package laid out like the reference's around it.
+
 Only tests/, bench.py's cpu_baseline / reference legs and tests/golden/make_golden.py may import
 this module.  The product package never does.
 """
@@ -117,3 +120,57 @@ def load_generator(mtc, fte, rescale=None):
                   if k == "src" or k.startswith("src.") or k.split(".")[0] in ("skimage", "matplotlib")]:
             del sys.modules[k]
         sys.modules.update(saved)
+
+
+def restated_generator(mtc, fte):
+    """load_generator's interface over the oracle's restatement of the glue (ms_oracle.get_costs,
+    extract_features_left / _lr, generate_test_cbmv), bound to `mtc` / `fte`.  The restatement is pinned
+    to the reference's stored outputs by tests/test_oracle_golden.py.  It has no generate_crop_train_cbmv."""
+    from oracle import ms_oracle as O
+
+    def get_default_args_dict():     # cbmv_generator.py:434-462, the entries generate_test_cbmv reads
+        return {"censw": 11, "nccw": 3, "sadw": 5, "sobelw": 5, "cens_sigma": 128.0, "ncc_sigma": 0.02,
+                "sad_sigma": 20000.0, "sobel_sigma": 20000.0, "ds_scale": 2}
+
+    def generate_test_cbmv(leftname, rightname, encoder_ds=64, maxdisp=192, args_dict=None, is_left_only=True):
+        import cv2
+        import torch
+        imgl, imgr = cv2.imread(leftname, 0), cv2.imread(rightname, 0)
+        f, h, w, ch, cw = O.generate_test_cbmv(imgl, imgr, encoder_ds, maxdisp, args_dict or get_default_args_dict(),
+                                               is_left_only, mtc=mtc, fte=fte)
+        return torch.from_numpy(f), h, w, ch, cw
+
+    return types.SimpleNamespace(
+        mtc=mtc, fte=fte, get_default_args_dict=get_default_args_dict, generate_test_cbmv=generate_test_cbmv,
+        get_costs=lambda *a: O.get_costs(*a, mtc=mtc, fte=fte),
+        extract_features_left=lambda *c: O.extract_features_left(*c, fte=fte),
+        extract_features_lr=lambda *c: O.extract_features_lr(*c, fte=fte))
+
+
+_STANDIN_GENERATOR = '''"""Stand-in for the reference's src/dataloader/cbmv_generator.py (oracle/ref_glue.py)."""
+import src.cpp.lib.libmatchers as mtc
+import src.cpp.lib.libfeatextract as fte
+from oracle import ref_glue as _ref_glue
+
+_g = _ref_glue.restated_generator(mtc, fte)
+get_default_args_dict = _g.get_default_args_dict
+get_costs = _g.get_costs
+extract_features_left = _g.extract_features_left
+extract_features_lr = _g.extract_features_lr
+generate_test_cbmv = _g.generate_test_cbmv
+'''
+
+
+def write_standin_package(root):
+    """Writes a package `src` under `root` laid out like the reference's: src/dataloader/cbmv_generator.py
+    imports `src.cpp.lib.libmatchers` / `libfeatextract` as cbmv_generator.py:16-17 do and serves its
+    functions from restated_generator().  Returns `root`, the directory to put on sys.path."""
+    files = {("src", "__init__.py"): "", ("src", "cpp", "__init__.py"): "",
+             ("src", "dataloader", "__init__.py"): "",
+             ("src", "dataloader", "cbmv_generator.py"): _STANDIN_GENERATOR}
+    for parts, text in files.items():
+        path = os.path.join(root, *parts)
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        with open(path, "w") as f:
+            f.write(text)
+    return root
