@@ -58,11 +58,7 @@ struct Win {
 
 // streaming (evict-first) stores for the write-once cost volumes
 __device__ __forceinline__ void st_stream(float* p, float v) { __stcs(p, v); }
-#ifdef MSN_EXP_NOSTG   // timing experiment only: the volume's stores never happen (the values are still computed)
-__device__ __forceinline__ void st_stream4(float* p, float4 v) { if (__float_as_uint(v.x) == 0x7fc00123u) __stcs(reinterpret_cast<float4*>(p), v); }
-#else
 __device__ __forceinline__ void st_stream4(float* p, float4 v) { __stcs(reinterpret_cast<float4*>(p), v); }
-#endif
 // bf16 volume (SURVEY.md 8f-4): the same values rounded to nearest even, four pixels per 64-bit store
 __device__ __forceinline__ void st_stream4(__nv_bfloat16* p, const float4& v) {
   const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);

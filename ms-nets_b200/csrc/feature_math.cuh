@@ -20,9 +20,6 @@ __device__ __forceinline__ float normalise_cost(float v, int matcher) {
 }
 
 __device__ __forceinline__ float ex2_approx(float x) {
-#ifdef MSN_EXP_NOMUFU   // timing experiment only (wrong results): what the SFU exponentials cost
-  return x * 0.5f;
-#endif
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;

@@ -273,7 +273,6 @@ struct FusedArgs {
   const float* first4;           // kModeRight: [N][4] raw costs that stand in where x + d >= w (get_right_cost's fill)
   float* first4_out;             // full mode, both views requested: where the left-view launch leaves those four
   int out_ch0;                   // first channel this launch writes (8 for the right view)
-  int tma_out;                   // channels 5-7 leave through the TMA engine (tile_back_half), see there
   const float* luts;    // [128] + [256], see ms_prep_kernel
   const float* sadsob;  // see FusedWs
   float* out;           // [N][8][D][h][w]
@@ -335,7 +334,7 @@ struct Lay : StageLay<DMAX, SLACK>, ParkLay<DMAX> {
   static constexpr size_t off_min = off_red + (size_t)kGroups * 4 * kTile * 4;    // [4][32]
   static constexpr size_t off_inv = off_min + 4 * kTile * 4;                      // [4][32]
   static constexpr size_t off_lut = off_inv + 4 * kTile * 4;                      // [128] census AML exponentials
-  static constexpr size_t off_lutn = off_lut + 128 * 4;                           // [256] census byte -> channel 0
+  static constexpr size_t off_lutn = off_lut + 128 * 4;                           // [256] census byte -> channel 0 (loaded, not read)
   static constexpr size_t off_par = (off_lutn + 256 * 4 + 127) & ~(size_t)127;    // 128 B aligned: TMA destination
   static constexpr size_t off_bar = off_par + P::pk_bytes;                        // 2 mbarriers
   static constexpr size_t bytes = off_bar + 32;
@@ -392,17 +391,6 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, i
           smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar)) : "memory");
 }
 
-// 3-D tiled tensor copy shared -> global (bulk async-group completion); elements outside the tensor are not written
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, const void* src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(map)), "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void tma_store_commit_and_wait_read() {   // shared memory may be reused / released after this
-  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-  asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-}
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
 // ---- packed fp32x2 arithmetic (Blackwell FADD2: two IEEE round-to-nearest adds per issue slot;
 //      operand B may be a scalar register broadcast to both halves, |x| is an operand modifier)
 typedef unsigned long long f32x2;
@@ -449,9 +437,6 @@ __device__ __forceinline__ f32x2 abs2(f32x2 v) {
   return pk2(fabsf(lo), fabsf(hi));
 }
 
-#ifdef MSN_EXP_NOPOPC   // timing experiment only (wrong results): what the census popcounts cost
-#define __popc(x) ((int)((x) & 31u))
-#endif
 struct TileId {
   int n, y, x0;   // y: row of the cropped image
   int yl;     // row inside this launch's band (output indexing)
@@ -603,10 +588,6 @@ struct P1State {
   float wv[5][6];      // sliding 5x6 right window; logical column j lives in wv[.][(j - 2*s) mod 6]
   int min_cen;
   float min_ncc, min_sad;
-#ifdef MSN_EXP_P1STORE   // timing experiment (clean blocks only): channels 1 and 3 leave the SM while phase 1 runs
-  float* optr;         // channel 1, row of the pair's first disparity, this thread's pixel (nullptr: pixel outside)
-  size_t oplane, ochan2;
-#endif
 };
 
 // One BLOCK of phase 1 = three disparity pairs (the rotation period of the window registers).
@@ -688,15 +669,6 @@ __device__ __forceinline__ void p1_block(P1State<L>& st, int dblk, int steps, in
     s_par[dsB * kTile + px] = nccB;
     s_par[2 * PS + dsA * kTile + px] = zA;
     s_par[2 * PS + dsB * kTile + px] = zB;
-#ifdef MSN_EXP_P1STORE
-    if (kClean && st.optr) {
-      st_stream(st.optr, normalise_cost(nccA, 1));
-      st_stream(st.optr + st.oplane, normalise_cost(nccB, 1));
-      st_stream(st.optr + st.ochan2, normalise_cost(zA, 3));
-      st_stream(st.optr + st.ochan2 + st.oplane, normalise_cost(zB, 3));
-    }
-    if (st.optr) st.optr += 2 * st.oplane;
-#endif
     st.min_cen = min(st.min_cen, min(cen_bA, cen_bB));
     st.min_ncc = fminf(st.min_ncc, fminf(nccA, nccB));
     st.min_sad = fminf(st.min_sad, fminf(zA, zB));
@@ -779,15 +751,6 @@ __device__ __forceinline__ Phase1Out phase1_tile(const FusedArgs& a, const TileI
   for (int r = 0; r < 5; ++r)
 #pragma unroll
     for (int j = 0; j < 6; ++j) st.wv[r][j] = st.rfp[r * L::RWF + j];
-#ifdef MSN_EXP_P1STORE
-  {
-    const size_t plane = (size_t)g.h * g.w, chan = plane * a.out_D;
-    st.oplane = plane; st.ochan2 = 2 * chan;
-    st.optr = (t.x0 + px < g.w) ? a.out + ((size_t)t.n * a.out_channels + a.out_ch0 + 1) * chan +
-                                      (size_t)(a.out_d0 + t.sub0 + d_lo) * plane + (size_t)t.yl * g.w + t.x0 + px
-                                : nullptr;
-  }
-#endif
   st.min_cen = 255;
   st.min_ncc = kFill;
   st.min_sad = kFill;
@@ -810,9 +773,6 @@ __device__ __forceinline__ Phase1Out phase1_tile(const FusedArgs& a, const TileI
         s_par[2 * PS + ds * kTile + px] = kFill;
       }
       st.rfp -= 6; st.dscp -= 6; st.ccp -= 6;   // (the window registers are never used again)
-#ifdef MSN_EXP_P1STORE
-      if (st.optr) st.optr += 6 * st.oplane;
-#endif
     } else {
       p1_block<L, false>(st, dblk, min(left, 6) >> 1, D, ap, l3, ld, ls, dmax_cen, dmax_ncc, dmax_sad, s_par, s_cen, px);
     }
@@ -1078,36 +1038,15 @@ __device__ __forceinline__ void finish_phase1(float* s_par, float* s_red, const 
   s_red[(grp * 4 + 3) * kTile + px] = o.min_sad;
 }
 
-// Census channels from a parked census byte (255 = no cost).  kCenLut: through the two shared-memory
-// tables (random indices: ~2.2 wavefronts per load); otherwise by arithmetic:
+// Census channels from a parked census byte (255 = no cost), by arithmetic:
 //  channel 0 = min(k,120)/120 as q = k*r, q' = fma(fma(-120, q, k), r, q) with r = fl(1/120): correctly
 //  rounded (= the true IEEE division NumPy does) for every k in 0..255, checked exhaustively in
-//  tests/test_host_math.py;  AML term = 2^(-(k-m)^2 k_cen), 0 for "no cost" -- what the table holds.
-#ifndef MSN_CEN_LUT
-#define MSN_CEN_LUT 1      // bit 0: denominator chain, bit 1: channel 0, bit 2: phase 3.  Measured at config B
-                           // (ms/pair): 0 -> 0.796, 1 -> 0.777 (the census chain is phase 2's critical path:
-                           // a table load is its cheapest step), 3 -> 0.787, 7 -> 0.786
-#endif
-constexpr bool kCenLutDen = (MSN_CEN_LUT & 1) != 0, kCenLutCh0 = (MSN_CEN_LUT & 2) != 0, kCenLutP3 = (MSN_CEN_LUT & 4) != 0;
-constexpr bool kCenLut = MSN_CEN_LUT != 0;
-#ifndef MSN_BACK_UNROLL
-#define MSN_BACK_UNROLL 1
-#endif
-constexpr int kBackUnroll = MSN_BACK_UNROLL;   // sweeps of phases 2/3 (measured: 1 is best)
-#ifndef MSN_P3_UNROLL
-#define MSN_P3_UNROLL MSN_BACK_UNROLL
-#endif
-constexpr int kP3Unroll = MSN_P3_UNROLL;
-#ifndef MSN_TMA_OUT
-#define MSN_TMA_OUT 0      // 1: build the TMA road for channels 5-7 (tile_back_half, kTmaOk); then MSNETS_TMA_OUT=1 selects it
-#endif
-constexpr bool kTmaOutBuilt = MSN_TMA_OUT != 0;
-#ifndef MSN_DEN_BATCH
-#define MSN_DEN_BATCH 8
-#endif
-constexpr int kDenBatch = MSN_DEN_BATCH;       // exponentials evaluated ahead of the denominator's dependent adds
-__device__ __forceinline__ float cen_ch0(int cb, const float* s_lutn) {
-  if (kCenLutCh0) return s_lutn[cb];
+//  tests/test_host_math.py;  AML term = 2^(-(k-m)^2 k_cen), 0 for "no cost".
+// Only the denominator chain takes the AML term from a shared-memory table instead (random indices: ~2.2
+// wavefronts per load).  Measured at config B (ms/pair): no table 0.796, table in the chain 0.777 (the census
+// chain is phase 2's critical path: a table load is its cheapest step), also for channel 0 0.787, also in
+// phase 3 0.786.
+__device__ __forceinline__ float cen_ch0(int cb) {
   const float k = (float)min(cb, 120);
   const float r = 1.0f / 120.0f;
   const float q = __fmul_rn(k, r);
@@ -1188,35 +1127,27 @@ __device__ __forceinline__ void store_quads(T* o, size_t chan, int nlive, const 
 // Channels 0-3 (cbmv_generator.py:283-287) for thread = (pixel quad q4, disparities d0, d0+16, ... < d1):
 // normalised costs stored as 128-bit row segments.
 template <bool kVec, class T>
-__device__ __forceinline__ void store_ch03(const float* s_par, const uint8_t* s_cen, const float* s_lutn, int PS,
-                                           int q4, int d0, int d1, T* orow, size_t plane, size_t chan,
-                                           int nlive) {
+__device__ __forceinline__ void store_ch03(const float* s_par, const uint8_t* s_cen, int PS, int q4, int d0, int d1,
+                                           T* orow, size_t plane, size_t chan, int nlive) {
   // (the output row is a pointer that advances by 16 planes per sweep: written as orow + d * plane, ptxas
   // redoes the 64-bit product every iteration -- ten more ALU-pipe instructions per four stores)
   T* o = orow + (size_t)d0 * plane;
   const size_t ostep = 16 * plane;
-#pragma unroll(kBackUnroll)
+#pragma unroll 1   // (measured: unrolling the back half's sweeps is slower)
   for (int d = d0; d < d1; d += 16, o += ostep) {
     const float* e0 = s_par + d * kTile + q4;
     const uint32_t cw = *reinterpret_cast<const uint32_t*>(s_cen + d * kTile + q4);
     const float4 v1 = *reinterpret_cast<const float4*>(e0);
     const float4 v2 = *reinterpret_cast<const float4*>(e0 + PS);
     const float4 v3 = *reinterpret_cast<const float4*>(e0 + 2 * PS);
-    float4 c0;
-    if (kCenLutCh0) c0 = make_float4(s_lutn[cw & 255u], s_lutn[(cw >> 8) & 255u], s_lutn[(cw >> 16) & 255u], s_lutn[cw >> 24]);
-    else c0 = cen_ch0_quad(cw);
+    const float4 c0 = cen_ch0_quad(cw);
     const float4 c1 = make_float4(normalise_cost(v1.x, 1), normalise_cost(v1.y, 1), normalise_cost(v1.z, 1),
                                   normalise_cost(v1.w, 1));
     const float4 c2 = make_float4(normalise_cost(v2.x, 2), normalise_cost(v2.y, 2), normalise_cost(v2.z, 2),
                                   normalise_cost(v2.w, 2));
     const float4 c3 = make_float4(normalise_cost(v3.x, 3), normalise_cost(v3.y, 3), normalise_cost(v3.z, 3),
                                   normalise_cost(v3.w, 3));
-#ifdef MSN_EXP_P1STORE
-    if (kVec) { st_stream4(o, c0); st_stream4(o + 2 * chan, c2); }
-    else store_quads<kVec>(o, chan, nlive, c0, c1, c2, c3);
-#else
     store_quads<kVec>(o, chan, nlive, c0, c1, c2, c3);
-#endif
   }
 }
 
@@ -1239,8 +1170,8 @@ __device__ __forceinline__ void p3_quad_exact(const float4& v, const float4& m, 
 
 // Channels 4-7 = exp(-(c-m)^2/sigma) / den for thread = (pixel quad q4, disparities dl, dl+32, ...),
 // exponentials recomputed from the parked costs, 128-bit row segments.
-template <bool kVec, class T, bool kExact = false, bool kTmaOut = false>
-__device__ __forceinline__ void phase3_quads(float* s_par, const uint8_t* s_cen, const float* s_lut,
+template <bool kVec, class T, bool kExact = false>
+__device__ __forceinline__ void phase3_quads(const float* s_par, const uint8_t* s_cen, const float* s_lut,
                                              const float* s_min, const float* s_inv, int PS, int q4, int dl, int D,
                                              T* arow, size_t plane, size_t chan, int nlive, float k0, float k1, float k2) {
   const float4 m_cen4 = *reinterpret_cast<const float4*>(s_min + q4);
@@ -1260,76 +1191,28 @@ __device__ __forceinline__ void phase3_quads(float* s_par, const uint8_t* s_cen,
   // census minima biased by 2^23 (exact: the minima are integers <= 120), see cen_bytes_as_biased_floats
   const f32x2 mp0[2] = {pk2(8388608.0f + (float)mcx, 8388608.0f + (float)mcy), pk2(8388608.0f + (float)mcz, 8388608.0f + (float)mcw)};
   const f32x2 ip0[2] = {pk2(i0.x, i0.y), pk2(i0.z, i0.w)};
-#ifdef MSN_P3_HALFWARPS   // A/B: phase 3 by warps 0-3 only (16 disparities per sweep), warps 4-7 leave the tile early
-  constexpr int kP3Step = 16;
-#else
-  constexpr int kP3Step = 32;
-#endif
-#pragma unroll(kP3Unroll)
-  for (int d = dl; d < D; d += kP3Step) {
-    float* e0 = s_par + d * kTile + q4;
-#ifdef MSN_EXP_NOP3LDS   // timing experiment only: phase 3 without its shared-memory reads
-    const float fd = (float)d;
-    const uchar4 cb = make_uchar4((unsigned char)d, (unsigned char)(d + 1), (unsigned char)(d + 2), (unsigned char)(d + 3));
-    const float4 v1 = make_float4(fd, fd + 1.f, fd + 2.f, fd + 3.f), v2 = make_float4(fd * 3.f, fd, fd + 5.f, fd), v3 = v1;
-#else
+#pragma unroll 1   // (measured: unrolling by 2 is slower)
+  for (int d = dl; d < D; d += 32) {
+    const float* e0 = s_par + d * kTile + q4;
     const uchar4 cb = *reinterpret_cast<const uchar4*>(s_cen + d * kTile + q4);
     const float4 v1 = *reinterpret_cast<const float4*>(e0);
     const float4 v2 = *reinterpret_cast<const float4*>(e0 + PS);
     const float4 v3 = *reinterpret_cast<const float4*>(e0 + 2 * PS);
-#endif
     float4 a0, a1, a2, a3;
-#ifdef MSN_EXP_NOP3COMPUTE   // timing experiment only: phase 3 stores what it loaded
-    if (!kExact) {
-      a0 = make_float4((float)cb.x, (float)cb.y, (float)cb.z, (float)cb.w); a1 = v1; a2 = v2; a3 = v3;
-      store_quads<kVec>(arow + (size_t)d * plane, chan, nlive, a0, a1, a2, a3);
-      continue;
-    }
-#endif
     if (kExact) {   // s_inv holds the denominators themselves (INFINITY where the pixel has no cost)
-      a0 = make_float4(__fdiv_rn(cen_e<kCenLutP3, true>(cb.x, mcx, s_lut, k0), i0.x), __fdiv_rn(cen_e<kCenLutP3, true>(cb.y, mcy, s_lut, k0), i0.y),
-                       __fdiv_rn(cen_e<kCenLutP3, true>(cb.z, mcz, s_lut, k0), i0.z), __fdiv_rn(cen_e<kCenLutP3, true>(cb.w, mcw, s_lut, k0), i0.w));
+      a0 = make_float4(__fdiv_rn(cen_e<false, true>(cb.x, mcx, s_lut, k0), i0.x), __fdiv_rn(cen_e<false, true>(cb.y, mcy, s_lut, k0), i0.y),
+                       __fdiv_rn(cen_e<false, true>(cb.z, mcz, s_lut, k0), i0.z), __fdiv_rn(cen_e<false, true>(cb.w, mcw, s_lut, k0), i0.w));
       p3_quad_exact(v1, m1, i1, -k1, a1);
       p3_quad_exact(v2, m2, i2, -k2, a2);
       p3_quad_exact(v3, m3, i3, -k2, a3);
     } else {
-      if (kCenLutP3) {
-        a0 = make_float4(cen_e<true>(cb.x, mcx, s_lut, k0) * i0.x, cen_e<true>(cb.y, mcy, s_lut, k0) * i0.y,
-                         cen_e<true>(cb.z, mcz, s_lut, k0) * i0.z, cen_e<true>(cb.w, mcw, s_lut, k0) * i0.w);
-      } else {
-        // (byte + 2^23) - (min + 2^23) = the integer difference cen_e squares; "no cost" is 65535 - min: exactly 0
-        p3_quad(cen_bytes_as_biased_floats<true>(*reinterpret_cast<const uint32_t*>(&cb)), mp0, ip0, nk0, a0);
-      }
+      // (byte + 2^23) - (min + 2^23) = the integer difference cen_e squares; "no cost" is 65535 - min: exactly 0
+      p3_quad(cen_bytes_as_biased_floats<true>(*reinterpret_cast<const uint32_t*>(&cb)), mp0, ip0, nk0, a0);
       p3_quad(v1, mp1, ip1, nk1, a1);
       p3_quad(v2, mp2, ip2, nk2, a2);
       p3_quad(v3, mp3, ip3, nk2, a3);
     }
-    if (kTmaOut) {
-      // channels 5-7 replace the parked costs they were made from (this thread is the only reader and writer of the
-      // quad); the tile's three planes leave through the TMA engine after the sweep.  Channel 4 has no float plane.
-      *reinterpret_cast<float4*>(e0) = a1;
-      *reinterpret_cast<float4*>(e0 + PS) = a2;
-      *reinterpret_cast<float4*>(e0 + 2 * PS) = a3;
-      T* o4 = arow + (size_t)d * plane;
-      if (kVec) st_stream4(o4, a0);
-      else {
-        const float c4[4] = {a0.x, a0.y, a0.z, a0.w};
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-          if (i < nlive) st_stream(o4 + i, c4[i]);
-      }
-    } else {
-      store_quads<kVec>(arow + (size_t)d * plane, chan, nlive, a0, a1, a2, a3);
-    }
-#ifdef MSN_FUSE_CH03   // A/B: channels 0-3 from the same loads in this sweep instead of warps 4-7 during the chain
-    {
-      const float4 c0 = cen_ch0_quad(*reinterpret_cast<const uint32_t*>(&cb));
-      const float4 c1 = make_float4(normalise_cost(v1.x, 1), normalise_cost(v1.y, 1), normalise_cost(v1.z, 1), normalise_cost(v1.w, 1));
-      const float4 c2 = make_float4(normalise_cost(v2.x, 2), normalise_cost(v2.y, 2), normalise_cost(v2.z, 2), normalise_cost(v2.w, 2));
-      const float4 c3 = make_float4(normalise_cost(v3.x, 3), normalise_cost(v3.y, 3), normalise_cost(v3.z, 3), normalise_cost(v3.w, 3));
-      store_quads<kVec>(arow - 4 * chan + (size_t)d * plane, chan, nlive, c0, c1, c2, c3);
-    }
-#endif
+    store_quads<kVec>(arow + (size_t)d * plane, chan, nlive, a0, a1, a2, a3);
   }
 }
 
@@ -1342,7 +1225,7 @@ __device__ __forceinline__ float den_chain(const FusedArgs& a, int warp, int lan
   constexpr int PS = L::PS;
   const int D = a.g.D;
   float den = 0.f;
-  constexpr int B = kDenBatch;
+  constexpr int B = 8;           // exponentials evaluated ahead of the denominator's dependent adds
   const int Dfull = D - D % B;   // groups of B without guards, then a guarded tail
   if (warp == 0) {
     const int mc = (mm == kFill) ? 0 : (int)mm;
@@ -1350,11 +1233,11 @@ __device__ __forceinline__ float den_chain(const FusedArgs& a, int warp, int lan
     for (int d0 = 0; d0 < Dfull; d0 += B, c += B * kTile) {
       float ev[B];
 #pragma unroll
-      for (int j = 0; j < B; ++j) ev[j] = cen_e<kCenLutDen, kExact>(c[j * kTile], mc, s_lut, a.k_cen);
+      for (int j = 0; j < B; ++j) ev[j] = cen_e<true, kExact>(c[j * kTile], mc, s_lut, a.k_cen);
 #pragma unroll
       for (int j = 0; j < B; ++j) den = __fadd_rn(den, ev[j]);
     }
-    for (int d = Dfull; d < D; ++d, c += kTile) den = __fadd_rn(den, cen_e<kCenLutDen, kExact>(c[0], mc, s_lut, a.k_cen));
+    for (int d = Dfull; d < D; ++d, c += kTile) den = __fadd_rn(den, cen_e<true, kExact>(c[0], mc, s_lut, a.k_cen));
   } else {
     const float kq = (warp == 1) ? a.k_ncc : a.k_sad;
     const f32x2 mm2 = pk2(mm, mm), nkq = pk2(-kq, -kq);
@@ -1459,7 +1342,7 @@ __device__ __forceinline__ void wta_scan(const FusedArgs& a, const TileId& t, in
     const uint8_t* c = s_cen + lane;
 #pragma unroll 4
     for (int d = 0; d < D; ++d) {
-      const float v = cen_ch0(c[d * kTile], nullptr);
+      const float v = cen_ch0(c[d * kTile]);
       if (v < m1) { m2 = m1; m1 = v; idx = d; }
       else if (v < m2) m2 = v;
     }
@@ -1497,16 +1380,10 @@ __device__ __forceinline__ void wta_scan(const FusedArgs& a, const TileId& t, in
 // part of the channel 0-3 stores to the chain warps statically or through a work counter (no
 // gain: the halves are already balanced), a warp-specialised persistent producer/consumer
 // kernel (15 % slower).
-// kTmaOk (the fp32 one-pass forms): when the launcher built a tensor map over the volume (a.tma_out), phase 3 writes
-// channels 5-7 over the parked costs they come from and one thread hands the three [D][32] planes to the TMA engine
-// (cp.async.bulk.tensor, shared -> global, clipped at the image edge).  Reason (profiles/micro/store_pattern.cu): an
-// SM's LSU store path takes about 32 bytes per clock, and both sweeps of the back half run exactly at that rate --
-// 98 KB in ~3 k cycles each; the bulk copies take another road.
-template <class L, bool kXchg, class T = float, bool kExact = false, bool kTmaOk = false>
+template <class L, bool kXchg, class T = float, bool kExact = false>
 __device__ __forceinline__ void tile_back_half(const FusedArgs& a, const TileId& t, long long tile, int tid,
-                                               float* s_par, const uint8_t* s_cen, float* s_red, float* s_min,
-                                               float* s_inv, const float* s_lut, const float* s_lutn,
-                                               const CUtensorMap* out_map = nullptr) {
+                                               const float* s_par, const uint8_t* s_cen, float* s_red, float* s_min,
+                                               float* s_inv, const float* s_lut) {
   constexpr int PS = L::PS;
   const FusedGeom& g = a.g;
   const int D = g.D;
@@ -1529,15 +1406,6 @@ __device__ __forceinline__ void tile_back_half(const FusedArgs& a, const TileId&
   T* orow = reinterpret_cast<T*>(a.out) + ((size_t)t.n * a.out_channels + a.out_ch0) * chan + (size_t)(a.out_d0 + t.sub0) * plane + (size_t)t.yl * g.w + (t.x0 + q4);
   const int nlive = min(4, g.w - (t.x0 + q4));  // live pixels of this quad (<= 0: none)
   const bool vec = vec_ok && nlive == 4;
-#ifdef MSN_EXP_SAMEADDR   // timing experiment only: every tile of an SM-resident pair of CTAs writes the SAME 8 x D row segments
-  orow = reinterpret_cast<T*>(a.out) + (size_t)(blockIdx.x % 296) * kTile + q4;   // (stays in L2: the stores cost no DRAM traffic)
-#endif
-#ifdef MSN_EXP_LINEAR   // timing experiment only (scrambled output): every tile writes ONE contiguous 8 x D x 128 B block
-  const size_t plane_x = kTile, chan_x = (size_t)D * kTile;
-  orow = reinterpret_cast<T*>(a.out) + (size_t)tile * 8 * D * kTile + q4;
-#define plane plane_x
-#define chan chan_x
-#endif
   if (warp < 4) {
     if (kXchg) {
       xchg_publish(a, 0, tile, t.v, warp, lane, s_inv);
@@ -1545,11 +1413,7 @@ __device__ __forceinline__ void tile_back_half(const FusedArgs& a, const TileId&
       bar_sync_128();
     }
     const float mm = kXchg ? s_min[warp * kTile + lane] : mm_own;
-#ifdef MSN_EXP_NOCHAIN   // timing experiment only: no denominator chain
-    float den = 1.0f + mm * 1e-30f;
-#else
     float den = den_chain<L, kExact>(a, warp, lane, mm, s_par, s_cen, s_lut);
-#endif
     if (kXchg) {
       s_red[warp * kTile + lane] = den;        // (the per-group minima are dead since the barrier above)
       bar_sync_128();
@@ -1562,39 +1426,14 @@ __device__ __forceinline__ void tile_back_half(const FusedArgs& a, const TileId&
   }
   else {
     // channels 0-3: thread = (pixel quad, d), 16 disparities per sweep of the four warps
-#if !defined(MSN_EXP_NOCH03) && !defined(MSN_FUSE_CH03)   // (NOCH03: timing experiment only, channels 0-3 never written)
-    if (vec) store_ch03<true>(s_par, s_cen, s_lutn, PS, q4, (tid >> 3) - 16, D, orow, plane, chan, nlive);
-    else store_ch03<false>(s_par, s_cen, s_lutn, PS, q4, (tid >> 3) - 16, D, orow, plane, chan, nlive);
-#endif
+    if (vec) store_ch03<true>(s_par, s_cen, PS, q4, (tid >> 3) - 16, D, orow, plane, chan, nlive);
+    else store_ch03<false>(s_par, s_cen, PS, q4, (tid >> 3) - 16, D, orow, plane, chan, nlive);
     if (a.wta_idx) wta_scan<L>(a, t, warp - 4, lane, s_par, s_cen);
   }
   __syncthreads();
-#ifdef MSN_EXP_NOP3      // timing experiment only: channels 4-7 are never written
-  return;
-#endif
-#ifdef MSN_P3_HALFWARPS
-  if (warp >= 4) return;
-#endif
   const int dl = tid >> 3;
-  if (kTmaOk && kTmaOutBuilt && a.tma_out) {
-    if (vec) phase3_quads<true, T, kExact, true>(s_par, s_cen, s_lut, s_min, s_inv, PS, q4, dl, D, orow + 4 * chan, plane, chan, nlive, a.k_cen, a.k_ncc, a.k_sad);
-    else phase3_quads<false, T, kExact, true>(s_par, s_cen, s_lut, s_min, s_inv, PS, q4, dl, D, orow + 4 * chan, plane, chan, nlive, a.k_cen, a.k_ncc, a.k_sad);
-    fence_proxy_async_smem();          // this thread's shared-memory writes -> visible to the async (TMA) proxy
-    __syncthreads();
-    if (tid == 0) {
-      const int z0 = (t.n * a.out_channels + a.out_ch0 + 5) * a.out_D + a.out_d0 + t.sub0;
-#pragma unroll
-      for (int m = 0; m < 3; ++m) tma_store_3d(out_map, s_par + m * PS, t.x0, t.yl, z0 + m * a.out_D);
-      tma_store_commit_and_wait_read();   // the CTA's shared memory must outlive the engine's reads
-    }
-    return;
-  }
   if (vec) phase3_quads<true, T, kExact>(s_par, s_cen, s_lut, s_min, s_inv, PS, q4, dl, D, orow + 4 * chan, plane, chan, nlive, a.k_cen, a.k_ncc, a.k_sad);
   else phase3_quads<false, T, kExact>(s_par, s_cen, s_lut, s_min, s_inv, PS, q4, dl, D, orow + 4 * chan, plane, chan, nlive, a.k_cen, a.k_ncc, a.k_sad);
-#ifdef MSN_EXP_LINEAR
-#undef plane
-#undef chan
-#endif
 }
 
 // Back half of a tile for DISPARITY-SLAB SHARDING (phase A of slab.cu, SURVEY.md 8e): the AML
@@ -1603,7 +1442,7 @@ __device__ __forceinline__ void tile_back_half(const FusedArgs& a, const TileId&
 // writes the slab's per-pixel minima; slab_phase_b/c finish the job after the all-reduces.
 template <class L>
 __device__ __forceinline__ void tile_slab_a(const FusedArgs& a, const TileId& t, int tid, const float* s_par,
-                                            const uint8_t* s_cen, const float* s_red, const float* s_lutn) {
+                                            const uint8_t* s_cen, const float* s_red) {
   constexpr int PS = L::PS;
   const FusedGeom& g = a.g;
   const int D = g.D;
@@ -1634,7 +1473,7 @@ __device__ __forceinline__ void tile_slab_a(const FusedArgs& a, const TileId& t,
     const float4 v3 = *reinterpret_cast<const float4*>(e0 + 2 * PS);
     const float4 v0 = make_float4(cb.x == 255 ? kFill : (float)cb.x, cb.y == 255 ? kFill : (float)cb.y,
                                   cb.z == 255 ? kFill : (float)cb.z, cb.w == 255 ? kFill : (float)cb.w);
-    const float4 c0 = make_float4(cen_ch0(cb.x, s_lutn), cen_ch0(cb.y, s_lutn), cen_ch0(cb.z, s_lutn), cen_ch0(cb.w, s_lutn));
+    const float4 c0 = make_float4(cen_ch0(cb.x), cen_ch0(cb.y), cen_ch0(cb.z), cen_ch0(cb.w));
     const float4 c1 = make_float4(normalise_cost(v1.x, 1), normalise_cost(v1.y, 1), normalise_cost(v1.z, 1),
                                   normalise_cost(v1.w, 1));
     const float4 c2 = make_float4(normalise_cost(v2.x, 2), normalise_cost(v2.y, 2), normalise_cost(v2.z, 2),
@@ -1674,8 +1513,7 @@ __device__ __forceinline__ void tile_slab_a(const FusedArgs& a, const TileId& t,
 // kMode: kModeFull the whole volume; kModeSlabA stop after phase 1 and emit what slab.cu's phase A emits
 // (tile_slab_a); kModeXchg a rank's disparity slab, minima and denominators traded inside the tile.
 template <int DMAX, bool kTma, int kMode>
-__device__ __forceinline__ void fused_tile(const FusedArgs& a, const CUtensorMap& sad_map, const CUtensorMap& out_map,
-                                           long long tile, int sub) {
+__device__ __forceinline__ void fused_tile(const FusedArgs& a, const CUtensorMap& sad_map, long long tile, int sub) {
   using L = Lay<DMAX, kSlack>;
   constexpr int NT = 256;
   constexpr int PS = L::PS;
@@ -1705,10 +1543,8 @@ __device__ __forceinline__ void fused_tile(const FusedArgs& a, const CUtensorMap
       mbar_init_fence();
       stage_rows_tma<L, true>(a, t, smem_raw, &s_bar[0]);
     }
-    if (kCenLut) {
-      if (tid < 128) s_lut[tid] = __ldg(a.luts + tid);
-      s_lutn[tid] = __ldg(a.luts + 128 + tid);
-    }
+    if (tid < 128) s_lut[tid] = __ldg(a.luts + tid);
+    s_lutn[tid] = __ldg(a.luts + 128 + tid);
     {
       const int Xr = t.x0 + px + g.bwl, Y = t.y + g.bh;
       const int dcrop = (g.w - 1 - (t.x0 + px)) - t.d0;
@@ -1729,7 +1565,7 @@ __device__ __forceinline__ void fused_tile(const FusedArgs& a, const CUtensorMap
     cp_async_wait_all();
     finish_right<L>(s_par, s_cen, s_red, ro, a.first4 + 4 * t.n, px, grp, d_lo, d_end);
     __syncthreads();
-    tile_back_half<L, false, float, false, true>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut, s_lutn, &out_map);
+    tile_back_half<L, false>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut);
     return;
   }
   if (kTma) {
@@ -1751,10 +1587,8 @@ __device__ __forceinline__ void fused_tile(const FusedArgs& a, const CUtensorMap
     for (int d = d_lo; d < d_end; ++d, src += splane, dst += kTile) cp_async4(dst, src);
     stage_right<L, NT>(a, t, smem_raw);
   }
-  if (kCenLut) {
-    if (tid < 128) s_lut[tid] = __ldg(a.luts + tid);
-    s_lutn[tid] = __ldg(a.luts + 128 + tid);
-  }
+  if (tid < 128) s_lut[tid] = __ldg(a.luts + tid);
+  s_lutn[tid] = __ldg(a.luts + 128 + tid);
   LeftRegs lr;
   load_left(a, t, px, lr);
   if (!kTma) cp_async_wait_all();
@@ -1772,159 +1606,22 @@ __device__ __forceinline__ void fused_tile(const FusedArgs& a, const CUtensorMap
       a.first4_out[4 * t.n + tid] = v;
     }
   }
-  if (kMode == kModeSlabA) tile_slab_a<L>(a, t, tid, s_par, s_cen, s_red, s_lutn);
-  else if (kMode == kModeExact) tile_back_half<L, false, float, true>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut, s_lutn);
-  else if (kMode == kModeBf16) tile_back_half<L, false, __nv_bfloat16>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut, s_lutn);
-  else if (kMode == kModeXchg) tile_back_half<L, true>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut, s_lutn);
-  else tile_back_half<L, false, float, false, true>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut, s_lutn, &out_map);
+  if (kMode == kModeSlabA) tile_slab_a<L>(a, t, tid, s_par, s_cen, s_red);
+  else if (kMode == kModeExact) tile_back_half<L, false, float, true>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut);
+  else if (kMode == kModeBf16) tile_back_half<L, false, __nv_bfloat16>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut);
+  else if (kMode == kModeXchg) tile_back_half<L, true>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut);
+  else tile_back_half<L, false>(a, t, tile, tid, s_par, s_cen, s_red, s_min, s_inv, s_lut);
 }
 
 template <int DMAX, bool kTma, int kMode>
 __global__ void __launch_bounds__(256, 2)
-ms_fused_kernel(const FusedArgs a, const __grid_constant__ CUtensorMap sad_map,
-                const __grid_constant__ CUtensorMap out_map) {
+ms_fused_kernel(const FusedArgs a, const __grid_constant__ CUtensorMap sad_map) {
   if (kMode == kModeXchg) {
     // CTA = (tile, sub-slab), sub-slab fastest: the CTAs that wait for each other's minima are dispatched
     // together.  A sub-slab is a virtual rank: its own disparity offset, its own row in the exchange tables.
-    fused_tile<DMAX, kTma, kMode>(a, sad_map, out_map, blockIdx.x / (unsigned)a.subs, (int)(blockIdx.x % (unsigned)a.subs));
+    fused_tile<DMAX, kTma, kMode>(a, sad_map, blockIdx.x / (unsigned)a.subs, (int)(blockIdx.x % (unsigned)a.subs));
   } else {
-    fused_tile<DMAX, kTma, kMode>(a, sad_map, out_map, blockIdx.x, 0);
-  }
-}
-
-
-// ---- disparity-slab exchange, two tiles per CTA ---------------------------------------------------------
-// A narrow slab (<= 96 disparities per CTA: eight GPUs on a 640-disparity frame hold 80 each) leaves a tile
-// too little work to hide the two trips its minima and denominators make to the other GPUs.  Here a CTA
-// owns TWO neighbouring tiles a, b of a row, each with its own parking and staging area, and interleaves
-// them so that every trip has real work to hide behind:
-//     phase 1(a) -> publish minima(a) -> phase 1(b) -> publish minima(b)
-//     warps 0-3:  collect minima(a), denominators(a), publish(a); the same for b; collect den(a), den(b)
-//     warps 4-7:  channels 0-3 of a and b (and the WTA by-product)
-//     phase 3(a), phase 3(b)
-// minima(a) travel during phase 1(b); den(a) travels while b's chain runs.  Same tables, same protocol as
-// the one-tile form (a rank may not mix the two, the launch geometry is part of the contract).
-template <int DMAX>
-struct Lay2 {
-  using S = StageLay<DMAX, kSlack>;
-  using P = ParkLay<DMAX>;
-  static constexpr int PS = P::PS;
-  static constexpr size_t off_stage0 = 0, off_stage1 = S::st_bytes;
-  static constexpr size_t off_red = 2 * S::st_bytes;                        // [8][4][32], transient, shared by a and b
-  static constexpr size_t off_small = off_red + (size_t)kGroups * 4 * kTile * 4;  // per tile: loc, min, den, tot, inv = 5 x [4][32]
-  static constexpr size_t small_bytes = 5 * 4 * kTile * 4;
-  static constexpr size_t off_lut = off_small + 2 * small_bytes;            // [128] + [256] census tables
-  static constexpr size_t off_par0 = (off_lut + 384 * 4 + 127) & ~(size_t)127;
-  static constexpr size_t off_par1 = off_par0 + P::pk_bytes;
-  static constexpr size_t off_bar = off_par1 + P::pk_bytes;                 // 4 mbarriers
-  static constexpr size_t bytes = off_bar + 64;
-  // what the shared helpers expect from a layout
-  static constexpr int kSl = S::kSl, RW = S::RW, RWF = S::RWF;
-  static constexpr size_t st_desc = S::st_desc, st_c = S::st_c, st_rf = S::st_rf;
-};
-
-template <int DMAX>
-__global__ void __launch_bounds__(256, 2)
-ms_slab_x2_kernel(const FusedArgs a, const __grid_constant__ CUtensorMap sad_map) {
-  using L = Lay2<DMAX>;
-  constexpr int PS = L::PS;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  const FusedGeom& g = a.g;
-  const int D = g.D;
-  const int tid = threadIdx.x, px = tid % kTile, grp = tid / kTile, warp = tid >> 5, lane = tid & 31;
-  const int d_lo = grp * a.DC, d_end = min(D, d_lo + a.DC);
-  const int sub = (int)(blockIdx.x % (unsigned)a.subs);
-  const unsigned pair = blockIdx.x / (unsigned)a.subs;
-  const int pairs_x = (a.tiles_x + 1) >> 1;
-  const int xp = (int)(pair % (unsigned)pairs_x);
-  const long long row = pair / (unsigned)pairs_x;                 // n * h + y
-  const long long tile_id[2] = {row * a.tiles_x + 2 * xp, row * a.tiles_x + 2 * xp + 1};
-  const int nt = (2 * xp + 1 < a.tiles_x) ? 2 : 1;
-  TileId tt[2];
-  tt[0] = decode_tile((int)tile_id[0], a, sub);
-  tt[1] = tt[0];
-  tt[1].x0 += kTile;
-  unsigned char* stage[2] = {smem_raw + L::off_stage0, smem_raw + L::off_stage1};
-  float* s_par[2] = {reinterpret_cast<float*>(smem_raw + L::off_par0), reinterpret_cast<float*>(smem_raw + L::off_par1)};
-  uint8_t* s_cen[2] = {smem_raw + L::off_par0 + L::P::pk_cen, smem_raw + L::off_par1 + L::P::pk_cen};
-  float* s_red = reinterpret_cast<float*>(smem_raw + L::off_red);
-  float* small[2] = {reinterpret_cast<float*>(smem_raw + L::off_small),
-                     reinterpret_cast<float*>(smem_raw + L::off_small + L::small_bytes)};
-  unsigned long long* s_bar = reinterpret_cast<unsigned long long*>(smem_raw + L::off_bar);
-  constexpr int kLoc = 0, kMin = 128, kDen = 256, kTot = 384, kInv = 512;   // offsets into small[i]
-  float* s_lut = reinterpret_cast<float*>(smem_raw + L::off_lut);
-  float* s_lutn = s_lut + 128;
-  if (kCenLut) {
-    if (tid < 128) s_lut[tid] = __ldg(a.luts + tid);
-    s_lutn[tid] = __ldg(a.luts + 128 + tid);
-  }
-  if (tid == 0) {
-    for (int i = 0; i < 4; ++i) mbar_init(&s_bar[i], 1);
-    mbar_init_fence();
-    for (int i = 0; i < nt; ++i) {
-      stage_rows_tma<L>(a, tt[i], stage[i], &s_bar[2 * i]);
-      stage_sad_tma(a, &sad_map, tt[i], s_par[i] + PS, &s_bar[2 * i + 1]);
-    }
-  }
-  __syncthreads();
-  for (int i = 0; i < nt; ++i) {
-    LeftRegs lr;
-    load_left(a, tt[i], px, lr);
-    mbar_wait(&s_bar[2 * i], 0);
-    const Phase1Out o = phase1_tile<L>(a, tt[i], stage[i], s_par[i], s_cen[i], lr, px, d_lo);
-    mbar_wait(&s_bar[2 * i + 1], 0);
-    finish_phase1<L>(s_par[i], s_red, o, px, grp, d_lo, d_end);
-    __syncthreads();
-    if (tid < 4 * kTile) {   // this slab's minima of tile i
-      float v = kFill;
-#pragma unroll
-      for (int gq = 0; gq < kGroups; ++gq) v = fminf(v, s_red[gq * 4 * kTile + tid]);
-      small[i][kLoc + tid] = v;
-    }
-    __syncthreads();         // (s_red is free for the next tile)
-    if (warp < 4) xchg_publish(a, 0, tile_id[i], tt[i].v, warp, lane, small[i] + kLoc);
-  }
-  const size_t plane = (size_t)g.h * g.w;
-  const size_t chan = plane * a.out_D;
-  const int q4 = (tid & 7) * 4;
-  const bool vec_ok = ((g.w & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.out) & 15) == 0);
-  float* orow[2];
-  int nlive[2];
-  for (int i = 0; i < 2; ++i) {
-    orow[i] = a.out + (size_t)tt[i].n * a.out_channels * chan + (size_t)(a.out_d0 + tt[i].sub0) * plane +
-              (size_t)tt[i].yl * g.w + (tt[i].x0 + q4);
-    nlive[i] = min(4, g.w - (tt[i].x0 + q4));
-  }
-  if (warp < 4) {
-    float mm[2] = {kFill, kFill};
-    for (int i = 0; i < nt; ++i) {
-      xchg_collect<false>(a, 0, tile_id[i], warp, lane, small[i] + kMin);
-      bar_sync_128();
-      mm[i] = small[i][kMin + warp * kTile + lane];
-      small[i][kDen + warp * kTile + lane] = den_chain<L>(a, warp, lane, mm[i], s_par[i], s_cen[i], s_lut);
-      bar_sync_128();
-      xchg_publish(a, 1, tile_id[i], tt[i].v, warp, lane, small[i] + kDen);
-    }
-    for (int i = 0; i < nt; ++i) {
-      xchg_collect<true>(a, 1, tile_id[i], warp, lane, small[i] + kTot);
-      bar_sync_128();
-      const float den = small[i][kTot + warp * kTile + lane];
-      small[i][kInv + warp * kTile + lane] = (mm[i] == kFill) ? 0.f : 1.0f / den;
-    }
-  } else {
-    for (int i = 0; i < nt; ++i) {
-      if (vec_ok && nlive[i] == 4) store_ch03<true>(s_par[i], s_cen[i], s_lutn, PS, q4, (tid >> 3) - 16, D, orow[i], plane, chan, nlive[i]);
-      else store_ch03<false>(s_par[i], s_cen[i], s_lutn, PS, q4, (tid >> 3) - 16, D, orow[i], plane, chan, nlive[i]);
-      if (a.wta_idx) wta_scan<L>(a, tt[i], warp - 4, lane, s_par[i], s_cen[i]);
-    }
-  }
-  __syncthreads();
-  const int dl = tid >> 3;
-  for (int i = 0; i < nt; ++i) {
-    if (vec_ok && nlive[i] == 4)
-      phase3_quads<true>(s_par[i], s_cen[i], s_lut, small[i] + kMin, small[i] + kInv, PS, q4, dl, D, orow[i] + 4 * chan, plane, chan, nlive[i], a.k_cen, a.k_ncc, a.k_sad);
-    else
-      phase3_quads<false>(s_par[i], s_cen[i], s_lut, small[i] + kMin, small[i] + kInv, PS, q4, dl, D, orow[i] + 4 * chan, plane, chan, nlive[i], a.k_cen, a.k_ncc, a.k_sad);
+    fused_tile<DMAX, kTma, kMode>(a, sad_map, blockIdx.x, 0);
   }
 }
 
@@ -1961,13 +1658,6 @@ static PFN_encodeTiled get_encode_fn() {
     return (PFN_encodeTiled)p;
   }();
   return fn;
-}
-// The two-tiles-per-CTA exchange kernel is opt-in (MSNETS_X2=1): measured slower than the one-tile form both with
-// local virtual ranks (width 80: 1.47 vs 1.32 ms per config-B pair equivalent) and across 8 GPUs (config M:
-// 12.1 vs 10.7 ms) -- two long phase-1 stretches per CTA overlap worse with the co-resident CTA than four short ones.
-static bool x2_disabled() {
-  const char* e = getenv("MSNETS_X2");
-  return !(e && e[0] == '1');
 }
 static bool tma_disabled() {
   const char* e = getenv("MSNETS_NO_TMA");
@@ -2006,48 +1696,10 @@ static bool sad_tensor_map(const FusedGeom& g, int H, int N, const float* base, 
   return true;
 }
 
-// 3-D tensor map over the output volume [planes = N*C*out_D][h][w] fp32, box 32 x 1 x D: one tile's [D][32] plane of a
-// channel (tile_back_half, kTmaOk).  Needs 16-byte aligned rows and base.
-static bool out_tensor_map(const float* base, int w, int h, long long planes, int D, CUtensorMap* out) {
-  if ((w & 3) || (reinterpret_cast<uintptr_t>(base) & 15) || D > 256 || planes > 2147483647LL) return false;
-  const MapKey key{base, w, h, (int)planes, D, 2};
-  {
-    std::lock_guard<std::mutex> lk(g_map_mu);
-    for (auto& kv : g_maps)
-      if (kv.first == key) {
-        *out = kv.second;
-        return true;
-      }
-  }
-  PFN_encodeTiled enc = get_encode_fn();
-  if (!enc) return false;
-  const cuuint64_t gdim[3] = {(cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)planes};
-  const cuuint64_t gstr[2] = {(cuuint64_t)w * 4, (cuuint64_t)h * w * 4};
-  const cuuint32_t box[3] = {(cuuint32_t)kTile, 1u, (cuuint32_t)D};
-  const cuuint32_t estr[3] = {1u, 1u, 1u};
-  if (enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), gdim, gstr, box, estr,
-          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-    return false;
-  std::lock_guard<std::mutex> lk(g_map_mu);
-  if (g_maps.size() >= 64) g_maps.erase(g_maps.begin());
-  g_maps.emplace_back(key, *out);
-  return true;
-}
-// Opt-in (a -DMSN_TMA_OUT=1 build, profiles/ab_variants.py, and MSNETS_TMA_OUT=1 at run time; the GPU suite passed
-// with it switched on, ragged right edge and both views included): measured at config B the TMA road is 1.2 % SLOWER (0.787 vs 0.778 ms per pair) although it
-// takes three of phase 3's four stores off the LSU path -- the sweep's time does not follow its store traffic any
-// more than its instruction count (DESIGN.md section 4) and the issuing thread's wait at the end of the tile costs.
-static bool tma_out_disabled() {
-  if (!kTmaOutBuilt) return true;   // (a -DMSN_TMA_OUT=1 build; the default library carries no code for it)
-  const char* e = getenv("MSNETS_TMA_OUT");
-  return !(e && e[0] == '1');
-}
-
 // One launch of an instantiation; the dynamic shared-memory opt-in is set once per instantiation
 // and device, not per launch.
 template <int DMAX, bool kTma, int kMode>
-static int launch_inst(const FusedArgs& a, const CUtensorMap& map, const CUtensorMap& omap, long long tiles, cudaStream_t s) {
+static int launch_inst(const FusedArgs& a, const CUtensorMap& map, long long tiles, cudaStream_t s) {
   auto kern = ms_fused_kernel<DMAX, kTma, kMode>;
   constexpr size_t smem = Lay<DMAX, kSlack>::bytes;
   static std::mutex mu;
@@ -2061,35 +1713,7 @@ static int launch_inst(const FusedArgs& a, const CUtensorMap& map, const CUtenso
       if (dev < 64) done_mask |= 1ull << dev;
     }
   }
-  if (const char* e = getenv("MSNETS_EXP_EXTRA_SMEM")) {   // experiment: extra dynamic shared memory = fewer CTAs per SM
-    const size_t big = smem + (size_t)atoi(e);
-    MSN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)big));
-    kern<<<(unsigned)(tiles * (kMode == kModeXchg ? a.subs : 1)), 256, big, s>>>(a, map, omap);
-    return 0;
-  }
-  kern<<<(unsigned)(tiles * (kMode == kModeXchg ? a.subs : 1)), 256, smem, s>>>(a, map, omap);
-  return 0;
-}
-
-template <int DMAX>
-static int launch_x2(const FusedArgs& a, const CUtensorMap& map, long long tiles, cudaStream_t s) {
-  auto kern = ms_slab_x2_kernel<DMAX>;
-  constexpr size_t smem = Lay2<DMAX>::bytes;
-  static std::mutex mu;
-  static unsigned long long done_mask = 0;
-  int dev = 0;
-  MSN_CUDA_OK(cudaGetDevice(&dev));
-  {
-    std::lock_guard<std::mutex> lk(mu);
-    if (dev >= 64 || !((done_mask >> dev) & 1ull)) {
-      MSN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      if (dev < 64) done_mask |= 1ull << dev;
-    }
-  }
-  const long long rows = tiles / a.tiles_x;
-  const long long ctas = rows * ((a.tiles_x + 1) / 2) * a.subs;
-  MSN_REQUIRE(ctas <= 2147483647LL, "ms_slab_fused: too many tiles for one launch");
-  kern<<<(unsigned)ctas, 256, smem, s>>>(a, map);
+  kern<<<(unsigned)(tiles * (kMode == kModeXchg ? a.subs : 1)), 256, smem, s>>>(a, map);
   return 0;
 }
 
@@ -2220,7 +1844,6 @@ int launch_ms_fused(const uint8_t* d_left, const uint8_t* d_right, int N, int H,
   a.wta_idx = nullptr; a.wta_min1 = a.wta_min2 = nullptr;
   if (wta && wta->idx) {
     MSN_REQUIRE(!d_mins && wta->min1 && wta->min2, "ms_features: the WTA by-product needs all three planes and the one-pass path");
-    MSN_REQUIRE(!kCenLutCh0, "ms_features: WTA by-product is built for the arithmetic channel-0 form");
     a.wta_idx = wta->idx; a.wta_min1 = wta->min1; a.wta_min2 = wta->min2;
   }
   memset(&a.xchg, 0, sizeof(a.xchg));
@@ -2245,32 +1868,13 @@ int launch_ms_fused(const uint8_t* d_left, const uint8_t* d_right, int N, int H,
   bool use_tma = g.D <= 256 && !tma_disabled();
   if (use_tma) use_tma = sad_tensor_map(g, H, N, ws.sadsob, &sad_map);
   a.DC = 2 * (((g.D + kGroups - 1) / kGroups + 1) / 2);   // phase 1 walks disparity pairs
-  // channels 5-7 (and 13-15) through the TMA engine: the fp32 one-pass forms
-  CUtensorMap out_map;
-  memset(&out_map, 0, sizeof(out_map));
-  a.tma_out = 0;
-  if (!exact && !out_bf16 && !xchg && !d_mins && !tma_disabled() && !tma_out_disabled() &&
-      out_tensor_map(d_out, g.w, g.h, (long long)N * a.out_channels * a.out_D, g.D, &out_map))
-    a.tma_out = 1;
-  // narrow exchange slabs: two tiles per CTA (ms_slab_x2_kernel)
-  if (xchg && use_tma && g.D <= 96 && !x2_disabled()) {
-    if (g.D <= 64) { if (launch_x2<64>(a, sad_map, tiles, s)) return 1; }
-    else { if (launch_x2<96>(a, sad_map, tiles, s)) return 1; }
-    MSN_LAUNCH_OK();
-    if (prof) {
-      MSN_CUDA_OK(cudaEventRecord(rec.ev[3], s));
-      std::lock_guard<std::mutex> lk(g_prof_mu);
-      g_prof.push_back(rec);
-    }
-    return 0;
-  }
 #define MSN_FUSED_LAUNCH(DMAX, TMA)                                                \
   {                                                                                \
-    if (exact) { if (launch_inst<DMAX, TMA, kModeExact>(a, sad_map, out_map, tiles, s)) return 1; } \
-    else if (out_bf16) { if (launch_inst<DMAX, TMA, kModeBf16>(a, sad_map, out_map, tiles, s)) return 1; } \
-    else if (xchg) { if (launch_inst<DMAX, TMA, kModeXchg>(a, sad_map, out_map, tiles, s)) return 1; } \
-    else if (d_mins) { if (launch_inst<DMAX, TMA, kModeSlabA>(a, sad_map, out_map, tiles, s)) return 1; } \
-    else { if (launch_inst<DMAX, TMA, kModeFull>(a, sad_map, out_map, tiles, s)) return 1; }    \
+    if (exact) { if (launch_inst<DMAX, TMA, kModeExact>(a, sad_map, tiles, s)) return 1; } \
+    else if (out_bf16) { if (launch_inst<DMAX, TMA, kModeBf16>(a, sad_map, tiles, s)) return 1; } \
+    else if (xchg) { if (launch_inst<DMAX, TMA, kModeXchg>(a, sad_map, tiles, s)) return 1; } \
+    else if (d_mins) { if (launch_inst<DMAX, TMA, kModeSlabA>(a, sad_map, tiles, s)) return 1; } \
+    else { if (launch_inst<DMAX, TMA, kModeFull>(a, sad_map, tiles, s)) return 1; }    \
   }
 #define MSN_FUSED_CASE(DMAX)                                                       \
   if (g.D <= DMAX) {                                                               \
@@ -2291,7 +1895,7 @@ int launch_ms_fused(const uint8_t* d_left, const uint8_t* d_right, int N, int H,
     a.first4_out = nullptr;
     a.out_ch0 = 8;
 #define MSN_RIGHT_CASE(DMAX) \
-  if (g.D <= DMAX) { if (launch_inst<DMAX, true, kModeRight>(a, sad_map, out_map, tiles, s)) return 1; } else
+  if (g.D <= DMAX) { if (launch_inst<DMAX, true, kModeRight>(a, sad_map, tiles, s)) return 1; } else
     MSN_RIGHT_CASE(64)
     MSN_RIGHT_CASE(128)
     MSN_RIGHT_CASE(192)

@@ -85,28 +85,24 @@ sadsob_vband_kernel(const float* __restrict__ L, const float* __restrict__ R, in
 // The same pre-pass for the fused path (compile-time pitch, zero-padded Sobel images), FOUR disparities per thread:
 // the column's L value is loaded once for the four, so a row costs 5 loads instead of 8 (the kernel is bound by
 // L1/L2 load throughput: every Sobel row is read once per disparity).  grid: (ceil(W/128), ceil(Dn/4), N).
-#ifndef MSN_VBAND_G
-#define MSN_VBAND_G 4
-#endif
-constexpr int kVbG = MSN_VBAND_G;
 template <int SP>
 __global__ void __launch_bounds__(128)
 sadsob_vbandg_kernel(const float* __restrict__ L, const float* __restrict__ R, int W, int d_begin, int Dn, int RB,
                      int NB, size_t img_stride, float* __restrict__ Vb) {
   const int IW = W + 1;
   const int j = blockIdx.x * blockDim.x + threadIdx.x + 1;
-  const int dd0 = blockIdx.y * kVbG, n = blockIdx.z;
+  const int dd0 = blockIdx.y * 4, n = blockIdx.z;
   if (j >= IW) return;
   const int jc = j - 1;
-  const int nk = min(kVbG, Dn - dd0);
+  const int nk = min(4, Dn - dd0);
   float* vb = Vb + (((size_t)n * Dn + dd0) * NB) * IW + j;       // disparity dd0 + k: + k * NB * IW
   const size_t kstride = (size_t)NB * IW;
   if (j == 1)
     for (int k = 0; k < nk; ++k)
       for (int b = 0; b < NB; ++b) vb[k * kstride + (size_t)b * IW - 1] = 0.f;
-  bool val[kVbG];
+  bool val[4];
 #pragma unroll
-  for (int k = 0; k < kVbG; ++k) val[k] = k < nk && jc >= d_begin + dd0 + k;   // else: left of the disparity, all zero
+  for (int k = 0; k < 4; ++k) val[k] = k < nk && jc >= d_begin + dd0 + k;   // else: left of the disparity, all zero
   if (!val[0]) {
     for (int k = 0; k < nk; ++k)
       for (int b = 0; b < NB; ++b) vb[k * kstride + (size_t)b * IW] = 0.f;
@@ -114,35 +110,35 @@ sadsob_vbandg_kernel(const float* __restrict__ L, const float* __restrict__ R, i
   }
   const float* l = L + n * img_stride + jc;
   const float* r = R + n * img_stride + (jc - d_begin - dd0);   // disparity dd0 + k reads r[-k] (r[0] where it has no column)
-  int roff[kVbG];
+  int roff[4];
 #pragma unroll
-  for (int k = 0; k < kVbG; ++k) roff[k] = val[k] ? -k : 0;
-  float v[kVbG];
+  for (int k = 0; k < 4; ++k) roff[k] = val[k] ? -k : 0;
+  float v[4];
 #pragma unroll
-  for (int k = 0; k < kVbG; ++k) v[k] = 0.f;
+  for (int k = 0; k < 4; ++k) v[k] = 0.f;
   for (int b = 0; b < NB; ++b, vb += IW) {
 #pragma unroll
-    for (int k = 0; k < kVbG; ++k)
+    for (int k = 0; k < 4; ++k)
       if (k < nk) vb[k * kstride] = v[k];
     if (b == NB - 1) break;
     int q0 = 0;
     for (; q0 + 3 <= RB; q0 += 3, l += 3 * SP, r += 3 * SP) {
-      float lv[3], rv[3][kVbG];
+      float lv[3], rv[3][4];
 #pragma unroll
       for (int q = 0; q < 3; ++q) {
         lv[q] = __ldg(l + q * SP);
 #pragma unroll
-        for (int k = 0; k < kVbG; ++k) rv[q][k] = __ldg(r + q * SP + roff[k]);
+        for (int k = 0; k < 4; ++k) rv[q][k] = __ldg(r + q * SP + roff[k]);
       }
 #pragma unroll
       for (int q = 0; q < 3; ++q)
 #pragma unroll
-        for (int k = 0; k < kVbG; ++k) v[k] = __fadd_rn(v[k], val[k] ? absdiff_rn(lv[q], rv[q][k]) : 0.f);
+        for (int k = 0; k < 4; ++k) v[k] = __fadd_rn(v[k], val[k] ? absdiff_rn(lv[q], rv[q][k]) : 0.f);
     }
     for (; q0 < RB; ++q0, l += SP, r += SP) {
       const float lq = __ldg(l);
 #pragma unroll
-      for (int k = 0; k < kVbG; ++k) v[k] = __fadd_rn(v[k], val[k] ? absdiff_rn(lq, __ldg(r + roff[k])) : 0.f);
+      for (int k = 0; k < 4; ++k) v[k] = __fadd_rn(v[k], val[k] ? absdiff_rn(lq, __ldg(r + roff[k])) : 0.f);
     }
   }
 }
@@ -575,7 +571,7 @@ int launch_sadsob5_padded(const float* L, const float* R, int N, int H, int W, i
   const size_t out_stride = (size_t)Dn * H * SP;
   dim3 g1(div_up(W, 128), Dn, N);
   (void)g1;
-  dim3 g4(div_up(W, 128), div_up(Dn, kVbG), N);
+  dim3 g4(div_up(W, 128), div_up(Dn, 4), N);
   if (SP == 1024) sadsob_vbandg_kernel<1024><<<g4, 128, 0, s>>>(L, R, W, d_begin, Dn, RB, NB, img_stride, Vb);
   else if (SP == 2048) sadsob_vbandg_kernel<2048><<<g4, 128, 0, s>>>(L, R, W, d_begin, Dn, RB, NB, img_stride, Vb);
   else sadsob_vbandg_kernel<4096><<<g4, 128, 0, s>>>(L, R, W, d_begin, Dn, RB, NB, img_stride, Vb);

@@ -138,10 +138,10 @@ def test_fused_slab_wta_parts_merge(oracle, world, D):
         x.close()
 
 
-def test_fused_slab_exchange_two_tiles_per_cta_form(oracle, monkeypatch):
-    """ms_slab_x2_kernel (opt-in, MSNETS_X2=1): narrow sub-slabs, two tiles per CTA, the same tables."""
+def test_fused_slab_exchange_narrow_sub_slabs(oracle, monkeypatch):
+    """The exchange kernel with slabs cut into sub-slabs at most 96 wide instead of 192: four of 96 disparities
+    at D = 384 on one rank, four of 80 per rank at D = 640 on two, beside slabs narrow enough to stay whole."""
     from msnets_b200 import sharding
-    monkeypatch.setenv("MSNETS_X2", "1")
     monkeypatch.setattr(sharding.ExchangeSlabMSFeatures, "TILE_D_CHOICES", (96,))
     for world, H, W, D in ((2, 36, 70, 40), (1, 34, 70, 384), (2, 30, 52, 640), (2, 34, 100, 128)):
         L, R = bordered_pair(H, W, 31 + world, border=10, patches=True)
