@@ -30,8 +30,10 @@ struct Vec<4> {
 // MODE 0: write disp; MODE 1: write partial (max, sum e, sum d*e) planes [N][3][HW];
 // MODE 2: input already holds probabilities -> plain expectation sum_d d*p_d
 // (the body of the reference's disparityregression, gcnet_3dcnn.py:136-139).
+// The float4 form is held to 3 CTAs (24 warps) per SM, the occupancy its loads in flight were measured at: left
+// alone, ptxas gives it 87 registers, which fits only 2.  The scalar form fits 6 CTAs in 40 registers.
 template <int V, int MODE>
-__global__ void __launch_bounds__(256)
+__global__ void __launch_bounds__(256, V == 4 ? 3 : 6)
 soft_argmin_kernel(const float* __restrict__ logits, int N, int D, long long HW, int d_begin,
                    float* __restrict__ out) {
   using VT = typename Vec<V>::T;
@@ -65,13 +67,18 @@ soft_argmin_kernel(const float* __restrict__ logits, int N, int D, long long HW,
 #pragma unroll
       for (int j = 0; j < kSaChunk; ++j)
         if (d0 + j < D) cm = fmaxf(cm, x[j][i]);
-      const float sc = ex2_approx((m[i] - cm) * kLog2e);  // first chunk: 2^-inf = 0
-      const float mlog = cm * kLog2e;
+      // While every logit so far is -inf (masked), subtract 0 so that (m, s, t) stays (-inf, 0, 0)
+      // instead of turning into 2^(-inf - -inf) = NaN.
+      const float cs = (cm == -INFINITY) ? 0.f : cm;
+      const float sc = ex2_approx((m[i] - cs) * kLog2e);  // first chunk: 2^-inf = 0
       float ss = s[i] * sc, tt = t[i] * sc;
 #pragma unroll
       for (int j = 0; j < kSaChunk; ++j)
         if (d0 + j < D) {
-          const float e = ex2_approx(fmaf(x[j][i], kLog2e, -mlog));
+          // x - max first: exact near the maximum (Sterbenz), so the weights do not depend on |max|.  Folding the
+          // shift into fma(x, log2e, -fl(max * log2e)) adds the rounding of that product, which grows with |max|
+          // and differs from chunk to chunk.
+          const float e = ex2_approx((x[j][i] - cs) * kLog2e);
           ss += e;
           tt = fmaf(e, (float)(d_begin + d0 + j), tt);
         }
@@ -127,7 +134,8 @@ soft_argmin_bwd_kernel(const float* __restrict__ logits, const float* __restrict
   for (int d = 0; d < D; ++d) {
     const float v = x[(size_t)d * HW];
     const float cm = fmaxf(m, v);
-    s = s * ex2_approx((m - cm) * kLog2e) + ex2_approx((v - cm) * kLog2e);
+    const float cs = (cm == -INFINITY) ? 0.f : cm;  // leading -inf logits: s stays 0, not NaN
+    s = s * ex2_approx((m - cs) * kLog2e) + ex2_approx((v - cs) * kLog2e);
     m = cm;
   }
   const float go = gout[(size_t)n * HW + p] / s, dv = disp[(size_t)n * HW + p];

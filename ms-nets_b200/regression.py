@@ -21,11 +21,24 @@ def _torch():
     return torch
 
 
-def _raw_soft_argmin(x, out=None):
+def _output(x, out, who):
+    """out= for a [N,D,H,W] input: a new tensor, or the caller's after checking it.  The kernels write
+    N*H*W floats through its raw pointer, so anything but a contiguous float32 [N,H,W] tensor on x's
+    device would be overrun or misread."""
     torch = _torch()
     N, D, H, W = x.shape
     if out is None:
-        out = torch.empty((N, H, W), dtype=torch.float32, device=x.device)
+        return torch.empty((N, H, W), dtype=torch.float32, device=x.device)
+    if (not isinstance(out, torch.Tensor) or tuple(out.shape) != (N, H, W) or out.dtype != torch.float32
+            or not out.is_contiguous() or out.device != x.device):
+        raise ValueError("%s: out must be a contiguous float32 [%d,%d,%d] tensor on %s" % (who, N, H, W, x.device))
+    return out
+
+
+def _raw_soft_argmin(x, out=None):
+    torch = _torch()
+    N, D, H, W = x.shape
+    out = _output(x, out, "soft_argmin")
     with torch.cuda.device(x.device):
         _lib.check(_lib.lib().msn_soft_argmin_dev(x.data_ptr(), N, D, H, W, out.data_ptr(),
                                                   torch.cuda.current_stream().cuda_stream))
@@ -35,8 +48,7 @@ def _raw_soft_argmin(x, out=None):
 def _raw_expected_disparity(x, out=None):
     torch = _torch()
     N, D, H, W = x.shape
-    if out is None:
-        out = torch.empty((N, H, W), dtype=torch.float32, device=x.device)
+    out = _output(x, out, "disparityregression")
     with torch.cuda.device(x.device):
         _lib.check(_lib.lib().msn_expect_disp_dev(x.data_ptr(), N, D, H, W, out.data_ptr(),
                                                   torch.cuda.current_stream().cuda_stream))
@@ -94,6 +106,7 @@ def _autograd_functions():
 
 def soft_argmin(logits, out=None):
     """logits: float32 [N,D,H,W] (CUDA tensor or NumPy array) -> disp float32 [N,H,W].
+    A -inf logit masks its disparity; a pixel masked at every disparity gives NaN, as torch's softmax does.
     Differentiable: when `logits` requires grad the result carries a grad_fn (backward =
     grad * softmax * (d - disp), msn_soft_argmin_backward_dev); `out=` is inference only."""
     if isinstance(logits, np.ndarray):
