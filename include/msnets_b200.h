@@ -295,6 +295,18 @@ MSN_API int msn_concat_volume_dev(const float* d_fl, const float* d_fr, int N, i
                           float* d_vol, void* stream);
 MSN_API int msn_diff_volume_dev(const float* d_fl, const float* d_fr, int N, int C, int H, int W, int D,
                         float* d_vol, void* stream);
+/* Backward of msn_concat_volume_dev: grad_vol [N][2C][D][H][W] -> grad_fl, grad_fr [N][C][H][W]:
+ *   grad_fl[n][c][y][x]  = sum over d = 0 .. min(x, D-1)      of grad_vol[n][c][d][y][x]
+ *   grad_fr[n][c][y][x'] = sum over d = 0 .. min(W-1-x', D-1) of grad_vol[n][C+c][d][y][x'+d]
+ * Each sum in fp32, d ascending from 0.0f, in one thread (deterministic, no atomics); masked voxels
+ * (x < d) never enter a sum, whatever they hold.  Either output may be NULL (not computed); not both.
+ * The concat form reads only the half of grad_vol that a non-NULL output needs. */
+MSN_API int msn_concat_volume_backward_dev(const float* d_grad_vol, int N, int C, int H, int W, int D,
+                                           float* d_grad_fl, float* d_grad_fr, void* stream);
+/* Backward of msn_diff_volume_dev: grad_vol [N][C][D][H][W] -> grad_fl, grad_fr [N][C][H][W], the concat
+ * sums taken over grad_vol[n][c] for both, grad_fr negated (same rules). */
+MSN_API int msn_diff_volume_backward_dev(const float* d_grad_vol, int N, int C, int H, int W, int D,
+                                         float* d_grad_fl, float* d_grad_fr, void* stream);
 
 #ifdef __cplusplus
 }

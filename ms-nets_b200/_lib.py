@@ -107,6 +107,8 @@ _SIGNATURES = {
     "msn_lrc_host": (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, _P]),
     "msn_concat_volume_dev": (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "msn_diff_volume_dev": (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    "msn_concat_volume_backward_dev": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P]),
+    "msn_diff_volume_backward_dev": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P]),
 }
 EXPORTS = tuple(sorted(_SIGNATURES))
 

@@ -1016,4 +1016,18 @@ int msn_diff_volume_dev(const float* d_fl, const float* d_fr, int N, int C, int 
   return launch_shift_volume(d_fl, d_fr, N, C, H, W, D, true, d_vol, as_stream(stream));
 }
 
+int msn_concat_volume_backward_dev(const float* d_grad_vol, int N, int C, int H, int W, int D, float* d_grad_fl,
+                                   float* d_grad_fr, void* stream) {
+  MSN_REQUIRE(d_grad_vol, "concat_volume_backward: null pointer argument");
+  MSN_REQUIRE(d_grad_fl || d_grad_fr, "concat_volume_backward: grad_fl and grad_fr are both NULL");
+  return launch_shift_volume_bwd(d_grad_vol, N, C, H, W, D, false, d_grad_fl, d_grad_fr, as_stream(stream));
+}
+
+int msn_diff_volume_backward_dev(const float* d_grad_vol, int N, int C, int H, int W, int D, float* d_grad_fl,
+                                 float* d_grad_fr, void* stream) {
+  MSN_REQUIRE(d_grad_vol, "diff_volume_backward: null pointer argument");
+  MSN_REQUIRE(d_grad_fl || d_grad_fr, "diff_volume_backward: grad_fl and grad_fr are both NULL");
+  return launch_shift_volume_bwd(d_grad_vol, N, C, H, W, D, true, d_grad_fl, d_grad_fr, as_stream(stream));
+}
+
 }  // extern "C"

@@ -142,5 +142,7 @@ int launch_soft_argmin_bwd(const float* logits, const float* disp, const float* 
 int launch_soft_argmin_merge(const float* parts, int P, int N, int H, int W, float* disp, cudaStream_t s);
 int launch_shift_volume(const float* fl, const float* fr, int N, int C, int H, int W, int D, bool diff,
                         float* vol, cudaStream_t s);
+int launch_shift_volume_bwd(const float* grad, int N, int C, int H, int W, int D, bool diff, float* gfl,
+                            float* gfr, cudaStream_t s);
 
 }  // namespace msn

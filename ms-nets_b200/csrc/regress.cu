@@ -270,4 +270,129 @@ int launch_shift_volume(const float* fl, const float* fr, int N, int C, int H, i
   return 0;
 }
 
+// Backward of the volumes above, G = d loss / d vol:
+// concat: gfl[n][c][y][x]  =   sum_{d=0..min(x, D-1)}     G[n][c][d][y][x]
+//         gfr[n][c][y][x'] =   sum_{d=0..min(W-1-x', D-1)} G[n][C+c][d][y][x'+d]
+// diff  : gfl as concat from G[n][c], gfr = -(the concat sum, taken over G[n][c] as well)
+// Every sum is in fp32, one rounding per add, d ascending from 0.0f, in one thread: no atomics and no split
+// of a sum across threads, so the result is deterministic and equals the NumPy restatement bit for bit.
+// A masked voxel (x < d, which covers every d >= W) never enters a sum, whatever it holds (NaN included);
+// the forward wrote 0 there.  diff negates the finished sum (the same bits as adding negated terms).
+//
+// One thread owns 4 consecutive columns x0..x0+3 of one (n, c, y) row, of gfl and of gfr, and walks d
+// kBwdChunk disparities at a time with every load of the chunk issued before the adds.  gfl: the aligned
+// quad at x0 of each plane, streamed once from HBM (__ldcs) in the concat form.  gfr needs columns x0+d ..
+// x0+d+3, the aligned quads k = d/4 and k+1 of the plane shifted by r = d % 4; d0 is a multiple of
+// kBwdChunk, so r is a compile-time constant in the unrolled chunk.  Those quads are what the neighbouring
+// threads of the warp (or the next warp) read at the same d, so across the grid every line of the
+// gradient volume is fetched from DRAM once and the diagonal re-reads come from L1 / L2.
+// The scalar form (W % 4 != 0 or a base pointer off 16 bytes) loads only the voxels it adds.
+constexpr int kBwdChunk = 4;
+
+template <bool kDiff, bool kVec>
+__global__ void __launch_bounds__(256)
+shift_volume_bwd_kernel(const float* __restrict__ g, int C, int H, int W, int D, float* __restrict__ gfl,
+                        float* __restrict__ gfr) {
+  static_assert(kBwdChunk % 4 == 0, "the gfr shift d % 4 must be a compile-time constant");
+  const int Wq = (W + 3) >> 2;
+  const long long row_groups = (long long)H * Wq;
+  const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= row_groups) return;
+  const int nc = blockIdx.y;  // n * C + ci
+  const int n = nc / C, ci = nc % C;
+  const int y = (int)(q / Wq), x0 = (int)(q % Wq) * 4;
+  const size_t plane = (size_t)H * W;
+  const int Cg = kDiff ? C : 2 * C;
+  const float* gl = g + ((size_t)n * Cg + ci) * D * plane + (size_t)y * W;   // plane 0 of G[n][c], row y
+  const float* gr = kDiff ? gl : gl + (size_t)C * D * plane;                 // plane 0 of G[n][C+c] (concat)
+  // sums of gfl run over d <= x (x <= x0+3), those of gfr over d <= W-1-x' (x' >= x0)
+  const int dl_end = gfl ? min(D, x0 + 4) : 0;
+  const int dr_end = gfr ? min(D, W - x0) : 0;
+  const int d_end = max(dl_end, dr_end);
+  float al[4] = {0.f, 0.f, 0.f, 0.f}, ar[4] = {0.f, 0.f, 0.f, 0.f};
+  for (int d0 = 0; d0 < d_end; d0 += kBwdChunk) {
+    float a[kBwdChunk][4], b[kBwdChunk][4];
+#pragma unroll
+    for (int j = 0; j < kBwdChunk; ++j) {
+      const int d = d0 + j;
+      const float* pl = gl + (size_t)d * plane;
+      const float* pr = gr + (size_t)d * plane;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) a[j][i] = b[j][i] = 0.f;
+      if (kVec) {
+        if (d < dl_end) {
+          const float4 v = kDiff ? __ldg(reinterpret_cast<const float4*>(pl + x0))
+                                 : __ldcs(reinterpret_cast<const float4*>(pl + x0));
+          a[j][0] = v.x; a[j][1] = v.y; a[j][2] = v.z; a[j][3] = v.w;
+        }
+        if (d < dr_end) {  // x0 + d < W: quad k holds column x0+d, so it lies inside the row
+          const int r = j & 3;
+          const int xk = x0 + (d - r);
+          const float4 u = __ldg(reinterpret_cast<const float4*>(pr + xk));
+          float w[8] = {u.x, u.y, u.z, u.w, 0.f, 0.f, 0.f, 0.f};
+          if (r != 0 && xk + 4 < W) {
+            const float4 t = __ldg(reinterpret_cast<const float4*>(pr + xk + 4));
+            w[4] = t.x; w[5] = t.y; w[6] = t.z; w[7] = t.w;
+          }
+#pragma unroll
+          for (int i = 0; i < 4; ++i) b[j][i] = w[r + i];
+        }
+      } else {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const int x = x0 + i;
+          if (d < dl_end && x >= d && x < W) a[j][i] = pl[x];
+          if (d < dr_end && x + d < W) b[j][i] = pr[x + d];
+        }
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < kBwdChunk; ++j) {
+      const int d = d0 + j;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int x = x0 + i;
+        if (d < dl_end && x >= d && x < W) al[i] += a[j][i];
+        if (d < dr_end && x + d < W) ar[i] += b[j][i];
+      }
+    }
+  }
+  const size_t o = ((size_t)nc * H + y) * W + x0;
+  if (kDiff) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) ar[i] = -ar[i];
+  }
+  if (kVec) {
+    if (gfl) *reinterpret_cast<float4*>(gfl + o) = make_float4(al[0], al[1], al[2], al[3]);
+    if (gfr) *reinterpret_cast<float4*>(gfr + o) = make_float4(ar[0], ar[1], ar[2], ar[3]);
+  } else {
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+      if (x0 + i < W) {
+        if (gfl) gfl[o + i] = al[i];
+        if (gfr) gfr[o + i] = ar[i];
+      }
+  }
+}
+
+int launch_shift_volume_bwd(const float* grad, int N, int C, int H, int W, int D, bool diff, float* gfl,
+                            float* gfr, cudaStream_t s) {
+  MSN_REQUIRE(N >= 0 && C >= 1 && H >= 0 && W >= 0 && D >= 1, "volume_backward: bad shape");
+  if (N == 0 || H == 0 || W == 0) return 0;
+  MSN_REQUIRE((long long)N * C <= 65535, "volume_backward: N*C too large for one launch");
+  auto aligned = [](const float* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+  const bool vec = (W & 3) == 0 && aligned(grad) && aligned(gfl) && aligned(gfr);   // NULL is aligned
+  // one thread per 4-column quad and all of its disparities: config P has 4.2 M quads per gradient
+  dim3 grid(div_up((long long)H * ((W + 3) / 4), 256), N * C);
+  if (diff) {
+    if (vec) shift_volume_bwd_kernel<true, true><<<grid, 256, 0, s>>>(grad, C, H, W, D, gfl, gfr);
+    else shift_volume_bwd_kernel<true, false><<<grid, 256, 0, s>>>(grad, C, H, W, D, gfl, gfr);
+  } else {
+    if (vec) shift_volume_bwd_kernel<false, true><<<grid, 256, 0, s>>>(grad, C, H, W, D, gfl, gfr);
+    else shift_volume_bwd_kernel<false, false><<<grid, 256, 0, s>>>(grad, C, H, W, D, gfl, gfr);
+  }
+  MSN_LAUNCH_OK();
+  return 0;
+}
+
 }  // namespace msn
